@@ -5,6 +5,7 @@
     python bench.py --gpus N --steps K --warmup W            # our arm (torchrun for N > 1)
     python bench.py --impl reference --gpus N --steps K ...   # CPU arm: the UNMODIFIED reference on host cores
     python bench.py --config 3|4|5|exact ...                  # the other BASELINE configs as the headline workload
+    python bench.py ... --dump-outputs DIR                    # + the last timed step's result rows, DIR/residuals.npy
 
 A step = one batch of R realizations (default 1000) of the whole 67-pulsar array through
 ``PulsarBatch.generate`` (throughput mode: in-kernel Philox; outputs stay in HBM).  ``value`` = realizations of
@@ -24,6 +25,7 @@ and without the collective).
 from __future__ import annotations
 
 import argparse
+import atexit
 import hashlib
 import json
 import os
@@ -38,6 +40,7 @@ sys.path.insert(0, ROOT)
 METRIC = "realizations/sec (67-psr ng15 GWB+RN+ECORR)"
 FALLBACK_HBM_GBS = 6650.0
 SEED = 20250922
+DUMP_BYTES = 60_000_000      # --dump-outputs writes at most this much (under 64 MB with the .npy header)
 NVLINK_PEER_GBS = 770.0      # B200_PROFILING.md: measured peer copy per direction per GPU (900 nominal)
 CGW3 = dict(gwtheta=1.5707963267948966, gwphi=2.5, mc=1e9, dist=5.0, fgw=1e-8, phase0=0.5, psi=1.5, inc=0.7853981633974483,
             pdist=1.0, psrTerm=True, evolve=True, tref=53000 * 86400)   # the reference test's source (tests/...:48-53)
@@ -80,6 +83,7 @@ class ClockSampler(threading.Thread):
             self.proc = subprocess.Popen(["nvidia-smi", f"--id={self.index}", f"--query-gpu={self.Q}",
                                           "--format=csv,noheader,nounits", "-lms", "100"],
                                          stdout=subprocess.PIPE, stderr=subprocess.DEVNULL, text=True)
+            atexit.register(self.proc.terminate)      # also when the run fails before finish(): no nvidia-smi left behind
             for line in self.proc.stdout:
                 if self.stop_flag:
                     break
@@ -228,8 +232,21 @@ def workload_name(cfg, kind, b, exact=False):
             + (", exact_epochs (one epoch per TOA: the literal F @ a)" if exact else ""))
 
 
-def timed_steps(b, R, steps, warmup, rc, world=1, rank=0, dist=None, k0=0):
-    """W untimed + K timed steps bracketed by barrier + synchronize; returns (ms max over ranks, per-kernel dict)."""
+def dump_outputs(dirpath, out):
+    """``--dump-outputs``: write ``dirpath/residuals.npy``, the rows (realizations) of ``out`` [rows, ld] (fp64, packed
+    engine order, as ``PulsarBatch.generate`` returns it) at a fixed, seeded choice of row indices; as many rows as fit in
+    DUMP_BYTES.  Same arguments, same rows: two builds can be compared output for output."""
+    import numpy as np
+    import torch
+    n_rows, ld = out.shape
+    rows = np.sort(np.random.default_rng(SEED).choice(n_rows, size=min(n_rows, DUMP_BYTES // (8 * ld)), replace=False))
+    os.makedirs(dirpath, exist_ok=True)
+    np.save(os.path.join(dirpath, "residuals.npy"), out[torch.from_numpy(rows).to(out.device)].cpu().numpy())
+
+
+def timed_steps(b, R, steps, warmup, rc, world=1, rank=0, dist=None, k0=0, dump=None):
+    """W untimed + K timed steps bracketed by barrier + synchronize; returns (ms max over ranks, per-kernel dict).
+    ``dump(out)`` (optional) receives the output buffer as the last timed step left it."""
     import numpy as np
     import torch
     out = getattr(b, "_bench_out", None)
@@ -256,6 +273,8 @@ def timed_steps(b, R, steps, warmup, rc, world=1, rank=0, dist=None, k0=0):
     if dist is not None:
         dist.barrier()
     ms = e0.elapsed_time(e1)
+    if dump is not None:
+        dump(out)
     timers = {}
     for k in range(steps):     # same K steps again with CUDA events around every launch (same stream, same schedule)
         step(warmup + steps + k, timers)
@@ -290,16 +309,18 @@ def short_line(b, R, rc, hbm, how, steps=3, warmup=2):
             "roofline_frac": rf["frac"], "whole_step_frac": rf["whole_step_frac"], "algorithmic_GBps": rf["achieved"]}
 
 
-def config5_block(args, world, rank, dist, hbm):
+def config5_block(args, world, rank, dist, hbm, steps=1, warmup=1, dump=None):
     """BASELINE config 5: 100k realizations of ng15-epoch strong-scaled over the ranks, final all-gather chunked
     (C realizations per rank per chunk) and overlapped with generation on a second stream; timed with and without
-    the collective on the identical schedule; one gathered chunk is checked bit for bit against local regeneration."""
+    the collective on the identical schedule (``warmup`` untimed + ``steps`` timed runs each; ms per run); one gathered
+    chunk is checked bit for bit against local regeneration.  ``dump(full)`` (optional) receives the gathered result of
+    the last timed run."""
     import torch
     from pta_replicator_b200 import distributed as D
     b, psrs, noise, setup_s, kind = make_batch("5", args)
     nreal, chunk = args.c5_nreal, args.c5_chunk
     C, n_chunks, padded = D.gather_plan(nreal, world, chunk)
-    full = torch.empty((padded, b.ld), dtype=torch.float64, device=b.device)
+    full = torch.zeros((padded, b.ld), dtype=torch.float64, device=b.device)   # the packed axis' alignment tail is never written
     comm = torch.cuda.Stream(b.device) if world > 1 else None
 
     def run(gather):
@@ -307,22 +328,26 @@ def config5_block(args, world, rank, dist, hbm):
 
     res = {}
     for gather in (False, True):
-        run(gather)                                   # warm-up (also creates the NCCL channels)
+        for _ in range(warmup):
+            run(gather)                               # warm-up (also creates the NCCL channels)
         torch.cuda.synchronize()
         if dist is not None:
             dist.barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         torch.cuda.synchronize()
         e0.record()
-        run(gather)
+        for _ in range(steps):
+            run(gather)
         e1.record()
         torch.cuda.synchronize()
         if dist is not None:
             dist.barrier()
-        t = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=b.device)
+        t = torch.tensor([e0.elapsed_time(e1) / steps], dtype=torch.float64, device=b.device)
         if dist is not None:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         res[gather] = float(t.item())
+    if dump is not None:
+        dump(full)
     p2p = None
     if world > 1:   # the same delivery by peer pushes (CUDA IPC + copy engines) instead of the NCCL collective
         try:
@@ -446,10 +471,15 @@ def main():
                     help="PulsarBatch(rn_taylor_tol=...): remainder bound of the in-epoch Taylor step, relative to the red-noise rms")
     ap.add_argument("--c5-nreal", type=int, default=100000)
     ap.add_argument("--c5-chunk", type=int, default=512)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed (rank 0's result rows, fp64, a fixed "
+                         "seeded sample of at most 60 MB) to DIR/residuals.npy")
     args = ap.parse_args()
     if args.bare:
         args.no_cpu = args.no_variants = args.no_extras = True
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs needs the GPU arm (--impl ours)")
         return run_reference(args)
 
     import torch
@@ -468,19 +498,17 @@ def main():
         # high-priority stream so their CTAs are scheduled as soon as generator CTAs retire
         os.environ.setdefault("TORCH_NCCL_HIGH_PRIORITY", "1")
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
-    if rank == 0 and not os.environ.get("PTAR_B200_LIB"):
-        ge.build()               # no-op when the in-tree .so is up to date
-    if dist is not None:
-        dist.barrier()           # the other ranks load the library only after rank 0 has (re)built it
+    # the library is the one build() compiled into the tree: nothing is compiled here (the tree may be read-only)
 
     cfg = "2" if args.config == "exact" else args.config
     exact = args.config == "exact"
     hbm, how = peaks()
+    dump = (lambda out: dump_outputs(args.dump_outputs, out)) if args.dump_outputs and rank == 0 else None
     if cfg == "5":               # config 5 as the headline: value = with the gather
-        blk = config5_block(args, world, rank, dist, hbm)
+        blk = config5_block(args, world, rank, dist, hbm, steps=args.steps, warmup=args.warmup, dump=dump)
         if rank == 0:
             print(json.dumps({"metric": METRIC, "value": blk["value_with_gather"], "unit": "realizations/s", "n_gpus": world,
-                              "steps": 1, "warmup": 1, "ms_per_step": blk["ms_with_gather"], "higher_is_better": True,
+                              "steps": args.steps, "warmup": args.warmup, "ms_per_step": blk["ms_with_gather"], "higher_is_better": True,
                               "scaling": "strong", "vs_baseline": None, "dtype": "f64", "data": "synthetic",
                               "config": {"workload": blk["workload"]}, "config5": blk}), flush=True)
         if dist is not None:
@@ -497,7 +525,7 @@ def main():
         t_wait = time.time()
         while not sampler.samples and time.time() - t_wait < 8.0:
             time.sleep(0.05)     # nvidia-smi can take a second to deliver its first sample
-    ms_max, kern, step = timed_steps(b, R, args.steps, args.warmup, args.rc, world, rank, dist)
+    ms_max, kern, step = timed_steps(b, R, args.steps, args.warmup, args.rc, world, rank, dist, dump=dump)
     if sampler:
         # the timed region lasts ~10-20 ms, shorter than nvidia-smi's 100 ms period: keep the identical load
         # running for ~0.7 s so that the clock / throttle record is taken under this load

@@ -21,6 +21,8 @@ and stores inputs + outputs as small npz files:
                     none of which the reference's own test covers (SURVEY.md section 4).
 ``ref_orf.npz``     ``spharmORFbasis.correlated_basis`` for lmax<=6 incl. coincident and
                     antipodal pairs.
+``ref_recipe8.npz`` one realization of the 15-yr recipe on 8 synthetic ng15-full pulsars
+                    (what ``oracle/recipe.py``, the numpy port, must reproduce).
 """
 from __future__ import annotations
 
@@ -360,6 +362,25 @@ def make_real(ref):
     np.savez_compressed(os.path.join(GOLD, "ref_real3.npz"), **out)
 
 
+RECIPE_STRIDE = 4   # every 4th TOA of each pulsar: keeps the fixture small (76k TOAs in all)
+
+
+def make_recipe(ref):
+    """One realization (seed 5) of the 15-yr recipe through the unmodified ``add_measurement_noise`` / ``add_jitter`` /
+    ``add_red_noise`` / ``add_gwb`` (oracle/refrecipe.py) on the first 8 pulsars of the synthetic ng15-full set: every
+    ``RECIPE_STRIDE``-th TOA of each pulsar and the rms of the whole realization per pulsar."""
+    from oracle import refrecipe
+    from pta_replicator_b200 import synthetic
+    psrs, noise = synthetic.make_ng15_like("full", npsr=8)
+    out = refrecipe.realization(refrecipe.dataset_from_pulsars(psrs, noise), 5)
+    store = {"npsr": np.array(len(out)), "seed": np.array(5), "stride": np.array(RECIPE_STRIDE)}
+    for i, d in enumerate(out):
+        store[f"delay_{i}"] = d[::RECIPE_STRIDE]
+        store[f"rms_{i}"] = np.array(np.sqrt(np.mean(d * d)))
+        store[f"ntoa_{i}"] = np.array(len(d))
+    np.savez_compressed(os.path.join(GOLD, "ref_recipe8.npz"), **store)
+
+
 def make_orf(ref):
     rng = np.random.default_rng(3)
     n = 9
@@ -391,6 +412,7 @@ def main():
     make_catalog(ref)
     make_f4(ref)
     make_outliers(ref)
+    make_recipe(ref)
     print("golden fixtures written to", GOLD)
 
 

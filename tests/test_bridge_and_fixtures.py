@@ -239,13 +239,15 @@ def test_oracle_on_the_real_ng15_files():
 
 def test_unmodified_reference_recipe_equals_the_port():
     """oracle/refrecipe.py (the UNMODIFIED functions under the stub harness: the CPU arm of bench.py) and
-    oracle/recipe.py (the numpy port) produce the same realization from the same seeds, 8 pulsars of ng15-full."""
-    from oracle import recipe, refrecipe, refstubs
+    oracle/recipe.py (the numpy port) produce the same realization from the same seeds, 8 pulsars of ng15-full.
+    The reference's side is tests/golden/ref_recipe8.npz (oracle/make_golden.py: every 4th TOA and the rms)."""
+    from oracle import recipe
     from pta_replicator_b200 import synthetic
-    if not refstubs.available():
-        pytest.skip("the reference is neither at /root/reference nor staged under oracle/_ref")
-    psrs, noise = synthetic.make_ng15_like("full", npsr=8)
-    a = refrecipe.realization(refrecipe.dataset_from_pulsars(psrs, noise), 5)
-    b = recipe.realization(recipe.dataset_from_pulsars(psrs, noise), 5)
-    worst = max(np.max(np.abs(x - y)) / np.sqrt(np.mean(y * y)) for x, y in zip(a, b))
+    z = np.load(os.path.join(GOLD, "ref_recipe8.npz"))
+    psrs, noise = synthetic.make_ng15_like("full", npsr=int(z["npsr"]))
+    b = recipe.realization(recipe.dataset_from_pulsars(psrs, noise), int(z["seed"]))
+    k = int(z["stride"])
+    assert [len(y) for y in b] == [int(z[f"ntoa_{i}"]) for i in range(len(b))]
+    worst = max(np.max(np.abs(z[f"delay_{i}"] - y[::k])) / np.sqrt(np.mean(y * y)) for i, y in enumerate(b))
     assert worst < 1e-13, worst
+    assert max(abs(float(z[f"rms_{i}"]) / np.sqrt(np.mean(y * y)) - 1.0) for i, y in enumerate(b)) < 1e-13

@@ -3,6 +3,9 @@ dictionary, the ORF closed form, ledger semantics, and that the C-ABI library lo
 every symbol include/ptar.h declares (no kernel is launched here)."""
 import os
 import re
+import subprocess
+import sys
+import textwrap
 
 import numpy as np
 import pytest
@@ -25,17 +28,24 @@ def test_cabi_exports_every_declared_symbol():
 
 
 def test_no_cpu_fallback_without_a_gpu():
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    import pta_replicator_b200 as P
-    from pta_replicator_b200 import _cabi
-    p = P.load_pulsar(os.path.join(GOLD, "partim_small", "par", "JPSR00.par"),
-                      os.path.join(GOLD, "partim_small", "tim", "fake_JPSR00_noiseonly.tim"))
-    P.make_ideal(p)
-    with pytest.raises(_cabi.PtarError, match="no CPU fallback"):
-        P.add_measurement_noise(p, efac=1.0)
-    assert p.added_signals == {}
+    """In a child process with every GPU hidden (CUDA_VISIBLE_DEVICES=""), so that it runs on GPU machines too."""
+    code = textwrap.dedent(f"""
+        import os
+        import pytest
+        import torch
+        assert not torch.cuda.is_available()
+        import pta_replicator_b200 as P
+        from pta_replicator_b200 import _cabi
+        p = P.load_pulsar(os.path.join({GOLD!r}, "partim_small", "par", "JPSR00.par"),
+                          os.path.join({GOLD!r}, "partim_small", "tim", "fake_JPSR00_noiseonly.tim"))
+        P.make_ideal(p)
+        with pytest.raises(_cabi.PtarError, match="no CPU fallback"):
+            P.add_measurement_noise(p, efac=1.0)
+        assert p.added_signals == {{}}
+    """)
+    r = subprocess.run([sys.executable, "-c", code], cwd=ROOT, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""),
+                       capture_output=True, text=True, timeout=600)
+    assert r.returncode == 0, r.stdout + r.stderr
 
 
 def test_product_does_not_import_the_oracle():
